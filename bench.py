@@ -46,7 +46,12 @@ def parse_args():
     ap.add_argument("--large-bodies", type=int, default=1_000_000, help="body count of the large pile in the configs block (the scene size BASELINE.json's north_star targets); 0 = skip it")
     ap.add_argument("--no-sharded", action="store_true", help="N > 1: skip the one-graph-over-N-GPUs block")
     ap.add_argument("--sharded-bodies", type=int, default=1_000_000, help="N > 1: body count of the pile whose single constraint graph is split over the N GPUs")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last timed step computed (body poses, velocities, world inverse "
+                    "inertias, accumulated impulses) as DIR/<name>.npy, so that two builds can be compared on identical inputs; rank 0 only")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def make_scene(args, seed):
@@ -57,6 +62,50 @@ def make_scene(args, seed):
     if args.scene == "ragdolls":
         return scenes.ragdolls(max(1, args.bodies // 16), seed=seed, motor=getattr(args, "ragdoll_motor", "motor"))
     return scenes.fallback_stress(args.bodies, hubs=max(1, args.bodies // 1000), seed=seed)
+
+
+DUMP_MAX_BODIES = 400_000  # 108 B per body in the dump
+DUMP_MAX_IMPULSES = 4 << 20  # floats: with the bodies, under 64 MiB in all
+
+
+def _sample(a, limit, seed):
+    """`a` itself when it has at most `limit` rows, otherwise the same seeded subset of rows on every run (kept in order)."""
+    if a.shape[0] <= limit:
+        return a
+    return a[np.sort(np.random.default_rng(seed).choice(a.shape[0], size=limit, replace=False))]
+
+
+def solve_outputs(sim):
+    """What a caller of Simulation.Solve reads back from `sim`'s host buffers: per body the pose, the velocity and the world inverse inertia (padding
+    floats dropped), and the accumulated impulses of every constraint, flattened in (batch, type batch, constraint, row) order."""
+    bodies = sim.bodies
+    impulses = [tb.accumulated_impulses.transpose(0, 2, 1).reshape(-1, tb.impulse_rows)[:tb.constraint_count].ravel() for tb in sim.type_batches()]
+    rows = _sample(np.arange(bodies.shape[0]), DUMP_MAX_BODIES, seed=1)
+    return {"body_poses": bodies[rows][:, 0:7].copy(), "body_velocities": bodies[rows][:, np.r_[8:11, 12:15]].copy(),
+            "body_world_inverse_inertias": bodies[rows][:, np.r_[16:23, 24:31]].copy(),
+            "accumulated_impulses": _sample(np.concatenate(impulses) if impulses else np.zeros(0, dtype=np.float32), DUMP_MAX_IMPULSES, seed=2)}
+
+
+def device_solve_outputs(ts, sim):
+    """solve_outputs of the state the last bepucuda_solve left on the device. The host buffers are restored afterwards, so that later uploads
+    from them send what they would have sent without the dump."""
+    kept_bodies = sim.bodies.copy()
+    type_batches = sim.type_batches()
+    kept_impulses = [tb.accumulated_impulses.copy() for tb in type_batches]
+    ts.download_bodies()
+    ts.download_impulses()
+    out = solve_outputs(sim)
+    sim.bodies[:] = kept_bodies
+    for tb, kept in zip(type_batches, kept_impulses):
+        tb.accumulated_impulses[:] = kept
+    return out
+
+
+def write_outputs(directory, outputs):
+    os.makedirs(directory, exist_ok=True)
+    for name, a in outputs.items():
+        assert a.dtype in (np.float32, np.float64)
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 def build_sim(args, seed):
@@ -314,7 +363,7 @@ def cpu_reference_run(args, steps, warmup, threads):
         ob.solve(sim, DT, threads=threads, simd=True)
     dt = time.perf_counter() - t0
     ci_per_step = sim.constraint_count * args.substeps * args.iterations
-    return {"value": ci_per_step * steps / dt, "ms_per_step": dt / steps * 1e3, "cores": threads, "constraints": sim.constraint_count, "description": desc}
+    return {"value": ci_per_step * steps / dt, "ms_per_step": dt / steps * 1e3, "cores": threads, "constraints": sim.constraint_count, "description": desc, "sim": sim}
 
 
 def run_reference_arm(args):
@@ -322,6 +371,8 @@ def run_reference_arm(args):
     if rank != 0:
         return
     r = cpu_reference_run(args, args.steps, args.warmup, args.cpu_threads)
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, solve_outputs(r["sim"]))
     line = {
         "impl": "reference", "metric": "constraint-iterations/sec (solver+integrator)", "value": r["value"], "unit": "constraint-iterations/s", "n_gpus": args.gpus,
         "steps": args.steps, "warmup": args.warmup, "ms_per_step": r["ms_per_step"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32",
@@ -403,6 +454,8 @@ def main():
     ci_per_step = int(t.constraint_iterations)
     launches_per_step = int(t.kernel_launches)
     alg_bytes_per_step = int(t.algorithmic_bytes)
+    if args.dump_outputs and rank == 0:
+        write_outputs(args.dump_outputs, device_solve_outputs(ts, sim))
 
     # ---- end to end through the C ABI with host buffers: H2D of bodies + prestep + impulses, solve, D2H of bodies + impulses ----
     for _ in range(2):

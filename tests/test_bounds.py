@@ -1,12 +1,11 @@
 """PredictBoundingBoxes on the device (SURVEY.md §8 f4, bepucuda_predict_bounding_boxes).
 
 CPU: the oracle's restatement (oracle_predict_bounding_boxes) reproduces, bit for bit, the committed known-answer vectors generated from the reference's
-own C# text (CapsuleWide / BoxWide / CylinderWide.GetBounds + BoundingBoxHelpers, transpiled: tests/golden/make_reference_bounds_vectors.py), fresh
-random inputs through the transpiled library when it is present, and closed-form answers (a sphere at rest, sleep-candidacy counting).
+own C# text (CapsuleWide / BoxWide / CylinderWide.GetBounds + BoundingBoxHelpers, transpiled: tests/golden/make_reference_bounds_vectors.py), the
+same library's recorded answers on fresh random inputs (tests/golden/make_reference_fresh_vectors.py), and closed-form answers (a sphere at rest, sleep-candidacy counting).
 GPU: the kernel is bit-identical to the oracle on random bodies of every supported shape, with the velocity callback, kinematic bodies, unsupported
 shapes, and on the body state a solve leaves resident."""
 import os
-import sys
 
 import numpy as np
 import pytest
@@ -67,19 +66,13 @@ def test_oracle_reproduces_the_reference_bounds_vectors_bit_for_bit(libs):
 
 
 def test_oracle_matches_the_transpiled_reference_on_fresh_inputs(libs):
-    sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
-    sys.path.insert(0, os.path.join(ROOT, "oracle", "ref_transpile"))
-    import build_ref
-    import make_reference_bounds_vectors as gen
-
-    if build_ref.build() is None:
-        pytest.skip("no reference tree and no prebuilt oracle/_ref here")
-    lib = gen.load_ref()
-    rng = np.random.default_rng(77)
-    inputs = gen.make_inputs(rng, 400)
-    want = gen.evaluate(lib, *inputs, DT)
-    got = _oracle_on_inputs(*inputs, DT)
-    assert np.array_equal(_bits(got[:, :7]), _bits(want))
+    """400 random bodies on another seed than the known-answer vectors; the transpiled library's bounds on them are recorded in
+    tests/golden/reference_fresh_vectors.npz (tests/golden/make_reference_fresh_vectors.py)."""
+    fresh = np.load(os.path.join(ROOT, "tests", "golden", "reference_fresh_vectors.npz"))
+    inputs = [fresh["bounds_" + name] for name in ("types", "dims", "margins", "allow", "q", "pos", "lin", "ang")]
+    assert inputs[0].shape == (400,)
+    got = _oracle_on_inputs(*inputs, float(fresh["bounds_dt"]))
+    assert np.array_equal(_bits(got[:, :7]), _bits(fresh["bounds_out"]))
 
 
 def test_known_answers_and_sleep_candidacy(libs):

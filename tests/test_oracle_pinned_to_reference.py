@@ -7,15 +7,16 @@ oracle/_ref/libbepu_ref.so, compiled without FMA contraction like RyuJIT's Vecto
   * committed known-answer vectors (tests/golden/reference_vectors.npz, generated from the transpiled reference by
     tests/golden/make_reference_vectors.py): every one of the 44 constraint types x {WarmStart, Solve, IncrementallyUpdateForSubstep}, the four
     PoseIntegration functions, and 38 chains of 1000 x (WarmStart; Solve) on the reference's constraint micro-benchmark inputs
-    (DemoBenchmarks/*ConstraintBenchmarks*.cs) -- these run anywhere, with or without /root/reference;
-  * live: when the reference tree (or a prebuilt oracle/_ref) is present, fresh random inputs through both libraries.
+    (DemoBenchmarks/*ConstraintBenchmarks*.cs);
+  * fresh inputs (tests/golden/reference_fresh_vectors.npz, recorded from the same library by tests/golden/make_reference_fresh_vectors.py):
+    32 more samples per type on other seeds, degenerate lanes among them.
+Both files are committed, so the checks run without the reference tree.
 
 What stays outside the pin: the solver driver (substep loop, batch order, integration responsibilities, gather/scatter, the TypeProcessor bundle
 loops), which is generic / unsafe C# the transpiler does not cover; tests/test_oracle.py holds those to closed-form answers.
 TEST INFRASTRUCTURE: nothing in the product loads either library."""
 import ctypes as C
 import os
-import sys
 
 import numpy as np
 import pytest
@@ -23,7 +24,6 @@ import pytest
 from oracle import binding as ob
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, os.path.join(ROOT, "oracle", "ref_transpile"))
 FP = C.POINTER(C.c_float)
 DT = 1.0 / 240.0
 
@@ -107,55 +107,47 @@ def test_oracle_reproduces_the_reference_benchmark_chains_bit_for_bit(oracle, go
 
 
 @pytest.fixture(scope="module")
-def reference_library():
-    import build_ref
-
-    path = build_ref.build()
-    if path is None:
-        pytest.skip("neither /root/reference nor a prebuilt oracle/_ref/libbepu_ref.so is present")
-    lib = C.CDLL(path)
-    lib.ref_eval_lane.argtypes = [C.c_int32, C.c_int32, FP, C.c_float, FP, FP, FP, C.c_int32]
-    lib.ref_eval_integration.argtypes = [C.c_int32, FP, FP]
-    lib.ref_covered_types.argtypes = [C.POINTER(C.c_int32), C.c_int32]
-    return lib
+def fresh():
+    """The transpiled reference's answers on the fresh inputs, recorded by tests/golden/make_reference_fresh_vectors.py."""
+    return np.load(os.path.join(ROOT, "tests", "golden", "reference_fresh_vectors.npz"))
 
 
-def test_transpiled_reference_covers_all_types_and_reproduces_the_committed_vectors(reference_library, golden):
-    ids = (C.c_int32 * 64)()
-    n = reference_library.ref_covered_types(ids, 64)
-    assert sorted(ids[:n]) == sorted(t for t in range(64) if ob.type_info(t) is not None)
-    key = "lane_07_"  # the committed file is what this library produces (regenerate with tests/golden/make_reference_vectors.py)
-    v, a, p = golden[key + "velocities"][0].copy(), golden[key + "impulses"][0].copy(), golden[key + "prestep"][0].copy()
-    assert reference_library.ref_eval_lane(7, 1, _ptr(np.ascontiguousarray(golden[key + "states"][0])), DT, _ptr(p), _ptr(a), _ptr(v), 1) == 0
-    assert np.array_equal(_bits(v), _bits(golden[key + "out1_velocities"][0]))
+def test_transpiled_reference_covers_all_types_and_reproduces_the_committed_vectors(oracle, golden, fresh):
+    assert sorted(fresh["covered_types"].tolist()) == sorted(t for t in range(64) if ob.type_info(t) is not None)
+    # both committed files come from the same library (regenerate them together with tests/golden/make_reference_vectors.py and
+    # tests/golden/make_reference_fresh_vectors.py)
+    assert np.array_equal(_bits(fresh["committed_lane_07_out1_velocities"]), _bits(golden["lane_07_out1_velocities"][0]))
 
 
-def test_oracle_matches_the_transpiled_reference_on_fresh_inputs(oracle, reference_library):
-    """Every type, every stage, 32 fresh samples per type (other seeds than the committed vectors), plus degenerate lanes: zero velocities and
-    impulses, identical poses, a kinematic partner (zero inverse mass and inertia)."""
-    from tests.test_device_source_on_host import _prestep_samples, _random_states
+def test_oracle_matches_the_transpiled_reference_on_fresh_inputs(oracle, fresh):
+    """Every type, every stage, 16 fresh samples per type (other seeds than the committed vectors), plus degenerate lanes: zero velocities and
+    impulses, identical poses, a kinematic partner (zero inverse mass and inertia). An output the file leaves out is the reference's input, unchanged."""
+    types = fresh["lane_types"].tolist()
+    assert types == sorted(t for t in range(64) if ob.type_info(t) is not None)
+    floats = {t: dict(zip(("states", "velocities", "impulses", "prestep"), (b * 14, b * 6, d, p))) for t, (b, p, d) in ((t, ob.type_info(t)) for t in types)}
 
-    samples = _prestep_samples()
-    rng = np.random.default_rng(991)
-    for type_id in sorted(samples):
-        bodies, prestep_rows, impulse_rows = ob.type_info(type_id)
-        for n, prestep in enumerate(samples[type_id]):
-            states = _random_states(rng, bodies)
-            vel = rng.normal(0, 1.5, (bodies, 6)).astype(np.float32)
-            imp = np.abs(rng.normal(0, 0.2, impulse_rows)).astype(np.float32)
-            if n % 8 == 5:
-                vel[:] = 0
-                imp[:] = 0
-            if n % 8 == 6 and bodies > 1:
-                states[1, 7:14] = 0  # kinematic partner
-            if n % 8 == 7:
-                states[:, 3:7] = (0, 0, 0, 1)
+    def split(name, among):
+        """The [16, floats per sample] blocks of the types `among` from the flat array lane_<name>."""
+        flat, out, at = fresh["lane_" + name], {}, 0
+        for t in among:
+            n = 16 * floats[t][name.split("_")[-1]]
+            out[t] = flat[at:at + n].reshape(16, -1)
+            at += n
+        assert at == flat.size, name
+        return out
+
+    given = {n: split(n, types) for n in ("states", "velocities", "impulses", "prestep")}
+    want = {}
+    for stage in (0, 1, 2):
+        for n in ("velocities", "impulses", "prestep"):
+            key = "lane_out%d_%s_types" % (stage, n)
+            changed = split("out%d_%s" % (stage, n), fresh[key].tolist()) if key in fresh.files else {}
+            want[(stage, n)] = {t: changed.get(t, given[n][t]) for t in types}
+    for type_id in types:
+        for i in range(16):
+            st = np.ascontiguousarray(given["states"][type_id][i])
             for stage in (0, 1, 2):
-                p1, a1, v1 = prestep.copy(), imp.copy(), vel.copy()
-                p2, a2, v2 = prestep.copy(), imp.copy(), vel.copy()
-                assert oracle.oracle_eval_lane(type_id, stage, _ptr(states), DT, _ptr(p1), _ptr(a1), _ptr(v1), 1) == 0
-                assert reference_library.ref_eval_lane(type_id, stage, _ptr(states), DT, _ptr(p2), _ptr(a2), _ptr(v2), 1) == 0
-                what = "type %d stage %d sample %d" % (type_id, stage, n)
-                assert np.array_equal(_bits(v1), _bits(v2)), what + ": velocities"
-                assert np.array_equal(_bits(a1), _bits(a2)), what + ": accumulated impulses"
-                assert np.array_equal(_bits(p1), _bits(p2)), what + ": prestep"
+                got = {n: given[n][type_id][i].copy() for n in ("velocities", "impulses", "prestep")}
+                assert oracle.oracle_eval_lane(type_id, stage, _ptr(st), DT, _ptr(got["prestep"]), _ptr(got["impulses"]), _ptr(got["velocities"]), 1) == 0
+                for n in got:
+                    assert np.array_equal(_bits(got[n]), _bits(want[(stage, n)][type_id][i])), "type %d stage %d sample %d: %s" % (type_id, stage, i, n)
