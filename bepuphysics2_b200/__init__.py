@@ -10,10 +10,11 @@ from .native import (  # noqa: F401
     BepuCudaError,
     CudaTimestepper,
     IntegratorDesc,
+    ShapeLibrary,
     Simulation,
     Timings,
     load_libraries,
     type_info,
 )
 
-__all__ = ["BepuCudaError", "CudaTimestepper", "IntegratorDesc", "Simulation", "Timings", "load_libraries", "type_info"]
+__all__ = ["BepuCudaError", "CudaTimestepper", "IntegratorDesc", "ShapeLibrary", "Simulation", "Timings", "load_libraries", "type_info"]

@@ -97,8 +97,8 @@ def build(force=False, verbose=False, variant=None, defines=()):
     flavours = [("fast", ["-DBEPU_NS=bepu_fast", "-prec-div=false", "-prec-sqrt=false"]), ("strict", ["-DBEPU_NS=bepu_strict", "-fmad=false"])]
     # (object, source, extra flags)
     units = [("solver_%s_%d.o" % (name, unit), "bepu_solver_kernels.cu", flags + ["-DBEPU_UNIT=%d" % unit]) for unit in (1, 0, 2, 3) for name, flags in flavours]
-    units += [("layout.o", "bepu_layout_kernels.cu", []), ("coloring.o", "bepu_coloring.cu", []), ("bounds.o", "bepu_bounds.cu", ["-fmad=false"]), ("api.o", "bepucuda_api.cu", [])]
-    all_sources = [os.path.join(CSRC, f) for f in ("bepu_solver_kernels.cu", "bepu_layout_kernels.cu", "bepu_coloring.cu", "bepu_bounds.cu", "bepucuda_api.cu")] + headers
+    units += [("layout.o", "bepu_layout_kernels.cu", []), ("coloring.o", "bepu_coloring.cu", []), ("bounds.o", "bepu_bounds.cu", ["-fmad=false"]), ("shape_bounds.o", "bepu_shape_bounds.cu", ["-fmad=false"]), ("api.o", "bepucuda_api.cu", [])]
+    all_sources = [os.path.join(CSRC, f) for f in ("bepu_solver_kernels.cu", "bepu_layout_kernels.cu", "bepu_coloring.cu", "bepu_bounds.cu", "bepu_shape_bounds.cu", "bepucuda_api.cu")] + headers
     # Nothing to compile when the library was built from exactly these sources (content stamp written after a build: survives a snapshot that
     # does not keep modification times) or is newer than every source. Object files need not travel with a snapshot.
     stamp = LIB_CUDA + ".stamp"

@@ -5,6 +5,7 @@
 #define BEPU_NS bepu_bounds_math
 #include "bepu_bounds_math.cuh"
 #include "bepu_bounds.h"
+#include "bepu_bounds_motion.cuh"
 
 namespace bepucuda {
 
@@ -16,30 +17,9 @@ __global__ void predict_bounding_boxes_kernel(BodyBuffers B, const BodyShape* __
                                               const __grid_constant__ PredictParams p) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= B.count) return;
-    const float4 q4 = B.pose[2 * (size_t)i], p4 = B.pose[2 * (size_t)i + 1];
-    const float4 l4 = B.velocity[2 * (size_t)i], w4 = B.velocity[2 * (size_t)i + 1];
-    const float4 i0 = B.inertia_local[2 * (size_t)i], i1 = B.inertia_local[2 * (size_t)i + 1];
-    const Q4 orientation = {q4.x, q4.y, q4.z, q4.w};
-    const V3 position = {p4.x, p4.y, p4.z};
-    Velocity velocity = {{l4.x, l4.y, l4.z}, {w4.x, w4.y, w4.z}};
-    // Bodies.IsKinematic (Bodies.cs:L326-331): every bit of inverse mass and inverse inertia is zero
-    const bool kinematic = (__float_as_uint(i1.z) | __float_as_uint(i0.x) | __float_as_uint(i0.y) | __float_as_uint(i0.z) | __float_as_uint(i0.w) | __float_as_uint(i1.x) | __float_as_uint(i1.y)) == 0u;
-    const bool integrate = p.integrate_velocity_for_kinematics != 0 || !kinematic;
-    const float sleepEnergy = length_squared(velocity.lin) + length_squared(velocity.ang);
-    // the integrated velocity is only used for the prediction; it is not stored (PoseIntegrator.cs:L339)
-    if (integrate) {
-        velocity.lin = (velocity.lin + V3{p.gravity_dt[0], p.gravity_dt[1], p.gravity_dt[2]}) * p.linear_damping_dt;
-        velocity.ang = velocity.ang * p.angular_damping_dt;
-    }
-    // UpdateSleepCandidacy (PoseIntegrator.cs:L286-304)
+    const PredictedMotion m = load_predicted_motion(B, i, p);
     BodyActivityRecord activity = activities[i];
-    if (sleepEnergy > activity.sleep_threshold) {
-        activity.timesteps_under_threshold_count = 0;
-        activity.sleep_candidate = 0;
-    } else if (activity.timesteps_under_threshold_count < 255) {
-        ++activity.timesteps_under_threshold_count;
-        if (activity.timesteps_under_threshold_count >= activity.minimum_timesteps_under_threshold) activity.sleep_candidate = 1;
-    }
+    update_sleep_candidacy(activity, m.sleep_energy);
     activities[i] = activity;
 
     const BodyShape shape = shapes[i];
@@ -51,7 +31,7 @@ __global__ void predict_bounding_boxes_kernel(BodyBuffers B, const BodyShape* __
     const ConvexShape convex = {shape.type, shape.a, shape.b, shape.c, shape.minimum_speculative_margin, shape.maximum_speculative_margin, shape.allow_expansion_beyond_speculative_margin};
     V3 bundleMin, bundleMax;
     float speculativeMargin;
-    convex_bounds(convex, orientation, position, velocity, p.dt, bundleMin, bundleMax, speculativeMargin);
+    convex_bounds(convex, m.orientation, m.position, m.velocity, p.dt, bundleMin, bundleMax, speculativeMargin);
     bounds[2 * (size_t)i] = make_float4(bundleMin.x, bundleMin.y, bundleMin.z, speculativeMargin);
     bounds[2 * (size_t)i + 1] = make_float4(bundleMax.x, bundleMax.y, bundleMax.z, 1.0f);
 }

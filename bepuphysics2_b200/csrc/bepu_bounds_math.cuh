@@ -56,21 +56,39 @@ BEPU_DI float angular_bounds_expansion(float angularSpeed, float dt, float maxim
     return fmin_ps(maximumAngularExpansion, sqrtf(-2.0f * maximumRadius * maximumRadius * cosAngleMinusOne));
 }
 
-// BoundingBoxBatcher.ExecuteConvexBatch for one body (BoundingBoxBatcher.cs:L176-197); `velocity` is the velocity AFTER the integration callback.
-BEPU_DI void convex_bounds(const ConvexShape& shape, Q4 orientation, V3 position, const Velocity& velocity, float dt, V3& bundleMin, V3& bundleMax, float& speculativeMargin) {
-    const LocalBounds local = shape_bounds(shape, orientation);
-    const float angularBoundsExpansion = angular_bounds_expansion(length(velocity.ang), dt, local.maximumRadius, local.maximumAngularExpansion);
+// BoundingBoxBatcher.ExecuteConvexBatch for one body (BoundingBoxBatcher.cs:L176-197), from the shape's local bounds onwards; `velocity` is the
+// velocity AFTER the integration callback. The margins are the ones of the body's collidable (also for a compound child: its parent's).
+BEPU_DI void expand_convex_bounds(V3 localMin, V3 localMax, float maximumRadius, float maximumAngularExpansion, float minimumSpeculativeMargin, float maximumSpeculativeMargin,
+                                  int32_t allowExpansionBeyondSpeculativeMargin, V3 position, const Velocity& velocity, float dt, V3& bundleMin, V3& bundleMax, float& speculativeMargin) {
+    const float angularBoundsExpansion = angular_bounds_expansion(length(velocity.ang), dt, maximumRadius, maximumAngularExpansion);
     speculativeMargin = length(velocity.lin) * dt + angularBoundsExpansion;
-    speculativeMargin = fmax_ps(shape.minimum_speculative_margin, fmin_ps(shape.maximum_speculative_margin, speculativeMargin));
-    const float maximumBoundsExpansion = shape.allow_expansion_beyond_speculative_margin ? 3.40282347e+38f : speculativeMargin;
+    speculativeMargin = fmax_ps(minimumSpeculativeMargin, fmin_ps(maximumSpeculativeMargin, speculativeMargin));
+    const float maximumBoundsExpansion = allowExpansionBeyondSpeculativeMargin ? 3.40282347e+38f : speculativeMargin;
     // BoundingBoxHelpers.GetBoundsExpansion (BoundingBoxHelpers.cs:L49-58)
     const V3 linearDisplacement = velocity.lin * dt;
     V3 minExpansion = {fmin_ps(0.0f, linearDisplacement.x) - angularBoundsExpansion, fmin_ps(0.0f, linearDisplacement.y) - angularBoundsExpansion, fmin_ps(0.0f, linearDisplacement.z) - angularBoundsExpansion};
     V3 maxExpansion = {fmax_ps(0.0f, linearDisplacement.x) + angularBoundsExpansion, fmax_ps(0.0f, linearDisplacement.y) + angularBoundsExpansion, fmax_ps(0.0f, linearDisplacement.z) + angularBoundsExpansion};
     minExpansion = {fmax_ps(-maximumBoundsExpansion, minExpansion.x), fmax_ps(-maximumBoundsExpansion, minExpansion.y), fmax_ps(-maximumBoundsExpansion, minExpansion.z)};
     maxExpansion = {fmin_ps(maximumBoundsExpansion, maxExpansion.x), fmin_ps(maximumBoundsExpansion, maxExpansion.y), fmin_ps(maximumBoundsExpansion, maxExpansion.z)};
-    bundleMin = position + ((-local.max) + minExpansion);
-    bundleMax = position + (local.max + maxExpansion);
+    bundleMin = position + (localMin + minExpansion);
+    bundleMax = position + (localMax + maxExpansion);
+}
+
+// The symmetric primitives (sphere, capsule, box, cylinder): local min = -max.
+BEPU_DI void convex_bounds(const ConvexShape& shape, Q4 orientation, V3 position, const Velocity& velocity, float dt, V3& bundleMin, V3& bundleMax, float& speculativeMargin) {
+    const LocalBounds local = shape_bounds(shape, orientation);
+    expand_convex_bounds(-local.max, local.max, local.maximumRadius, local.maximumAngularExpansion, shape.minimum_speculative_margin, shape.maximum_speculative_margin,
+                         shape.allow_expansion_beyond_speculative_margin, position, velocity, dt, bundleMin, bundleMax, speculativeMargin);
+}
+
+// DemoPoseIntegratorCallbacks.IntegrateVelocity (Demos/DemoCallbacks.cs:L99-104) on a copy of the velocity: PredictBoundingBoxes bounds the body
+// with the integrated velocity but does not store it (PoseIntegrator.cs:L339). Every bounds kernel goes through this one function.
+BEPU_DI Velocity predicted_velocity(Velocity velocity, bool integrate, const float gravityDt[3], float linearDampingDt, float angularDampingDt) {
+    if (integrate) {
+        velocity.lin = (velocity.lin + V3{gravityDt[0], gravityDt[1], gravityDt[2]}) * linearDampingDt;
+        velocity.ang = velocity.ang * angularDampingDt;
+    }
+    return velocity;
 }
 
 }  // namespace BEPU_NS

@@ -13,6 +13,7 @@
 #include "bepu_layout_kernels.h"
 #include "bepu_coloring.h"
 #include "bepu_bounds.h"
+#include "bepu_shape_bounds.h"
 
 using namespace bepucuda;
 
@@ -215,6 +216,22 @@ struct bepucuda_ctx {
     cudaEvent_t user_events[16] = {};
     DeviceBuffer body_shapes, body_activities, body_bounds;  // bepucuda_set_body_shapes / bepucuda_predict_bounding_boxes
     int shape_count = -1;
+    // bepucuda_set_shape_library / bepucuda_set_body_collidables
+    struct ShapeBounds {
+        DeviceBuffer library[12];  // the arrays of bepucuda_shape_library, in its field order
+        ShapeLibraryView view{};
+        bool library_set = false;
+        bepucuda_shape_library counts{};  // counts only (pointers cleared)
+        std::vector<bepucuda_mesh> meshes;
+        DeviceBuffer collidables, hull_bodies, compound_bodies, mesh_bodies, mesh_chunks, mesh_partials;
+        ShapeBoundsWork work{};
+        int collidable_count = -1;
+        bool active = false;  // set_body_collidables was called after set_body_shapes
+        void release() {
+            for (auto& b : library) b.release();
+            for (DeviceBuffer* b : {&collidables, &hull_bodies, &compound_bodies, &mesh_bodies, &mesh_chunks, &mesh_partials}) b->release();
+        }
+    } shape_bounds;
     DeviceBuffer color_refs, color_priorities, color_body_min, color_body_mask, color_out, color_lists, color_counts;  // bepucuda_color_constraints
     std::vector<cudaEvent_t> profile_events;
 };
@@ -578,6 +595,7 @@ int32_t bepucuda_destroy(bepucuda_ctx* ctx) {
                             &ctx->sync_mask, &ctx->chunk_table, &ctx->record_table, &ctx->ref_rows, &ctx->body_shapes, &ctx->body_activities, &ctx->body_bounds, &ctx->color_refs, &ctx->color_priorities, &ctx->color_body_min, &ctx->color_body_mask, &ctx->color_out, &ctx->color_lists, &ctx->color_counts, &ctx->source_bundle_flags, &ctx->refs32, &ctx->prestep32, &ctx->impulses32, &ctx->tb_table, &ctx->tdesc_table, &ctx->work_table, &ctx->map_table,
                             &ctx->bodies_per_type, &ctx->kinematics_dev, &ctx->program_dev, &ctx->frame_params_dev, &ctx->error_dev, &ctx->exchange_staging};
     for (auto b : bufs) b->release();
+    ctx->shape_bounds.release();
     ctx->raw_arena.release();
     ctx->pinned_arena.release();
     if (ctx->frame_params_host) cudaFreeHost(ctx->frame_params_host);
@@ -1453,12 +1471,16 @@ int32_t bepucuda_set_body_shapes(bepucuda_ctx* ctx, const bepucuda_body_shape* s
     if (body_count > 0) CK(cudaMemcpyAsync(ctx->body_shapes.ptr, shapes, (size_t)body_count * sizeof(BodyShape), cudaMemcpyHostToDevice, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));  // the caller's buffer is only guaranteed for the duration of the call
     ctx->shape_count = body_count;
+    ctx->shape_bounds.active = false;
     return BEPUCUDA_OK;
 }
 
 int32_t bepucuda_predict_bounding_boxes(bepucuda_ctx* ctx, float dt, bepucuda_body_activity* activities, float* bounds_out) {
     if (!ctx || !(dt > 0) || !activities || !bounds_out) return fail(ctx, BEPUCUDA_ERR_INVALID_ARGUMENT, "predict_bounding_boxes: bad arguments");
-    if (ctx->shape_count != ctx->body_count) return fail(ctx, BEPUCUDA_ERR_BAD_STATE, "predict_bounding_boxes: bepucuda_set_body_shapes was not called for the current body count");
+    auto& sb = ctx->shape_bounds;
+    if (sb.active && sb.collidable_count != ctx->body_count)
+        return fail(ctx, BEPUCUDA_ERR_BAD_STATE, "predict_bounding_boxes: bepucuda_set_body_collidables was not called for the current body count");
+    if (!sb.active && ctx->shape_count != ctx->body_count) return fail(ctx, BEPUCUDA_ERR_BAD_STATE, "predict_bounding_boxes: bepucuda_set_body_shapes was not called for the current body count");
     const int n = ctx->body_count;
     if (n == 0) return BEPUCUDA_OK;
     CK(cudaSetDevice(ctx->device));
@@ -1473,11 +1495,174 @@ int32_t bepucuda_predict_bounding_boxes(bepucuda_ctx* ctx, float dt, bepucuda_bo
     p.linear_damping_dt = powf(clamp01(1 - ctx->integ.linear_damping), dt);
     p.angular_damping_dt = powf(clamp01(1 - ctx->integ.angular_damping), dt);
     p.integrate_velocity_for_kinematics = ctx->integ.integrate_velocity_for_kinematics;
-    launch_predict_bounding_boxes(ctx->B, ctx->body_shapes.as<BodyShape>(), ctx->body_activities.as<BodyActivityRecord>(), ctx->body_bounds.as<float4>(), p, ctx->stream);
+    if (sb.active)
+        launch_predict_shape_bounds(ctx->B, sb.view, sb.work, ctx->body_activities.as<BodyActivityRecord>(), ctx->body_bounds.as<float4>(), p, ctx->stream);
+    else
+        launch_predict_bounding_boxes(ctx->B, ctx->body_shapes.as<BodyShape>(), ctx->body_activities.as<BodyActivityRecord>(), ctx->body_bounds.as<float4>(), p, ctx->stream);
     CK(cudaGetLastError());
     CK(cudaMemcpyAsync(activities, ctx->body_activities.ptr, (size_t)n * sizeof(BodyActivityRecord), cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaMemcpyAsync(bounds_out, ctx->body_bounds.ptr, (size_t)n * 32, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
+    return BEPUCUDA_OK;
+}
+
+static_assert(sizeof(bepucuda_hull) == sizeof(bepu_bounds_math::HullRecord) && sizeof(bepucuda_compound) == sizeof(bepu_bounds_math::CompoundRecord) &&
+                  sizeof(bepucuda_compound_child) == 32 && sizeof(bepucuda_compound_child) == sizeof(bepu_bounds_math::CompoundChildRecord) &&
+                  sizeof(bepucuda_mesh) == sizeof(bepu_bounds_math::MeshRecord) && sizeof(bepucuda_body_collidable) == sizeof(BodyCollidableRecord),
+              "ABI structs mirror the device records");
+
+namespace {
+// Element count of a library shape type (0 for a type the library does not hold).
+int64_t library_count(const bepucuda_shape_library& l, int32_t type) {
+    switch (type) {
+        case 0: return l.sphere_count;
+        case 1: return l.capsule_count;
+        case 2: return l.box_count;
+        case 3: return l.triangle_count;
+        case 4: return l.cylinder_count;
+        case 5: return l.hull_count;
+        case 6: return l.compound_count;
+        case 7: return l.big_compound_count;
+        case 8: return l.mesh_count;
+        default: return 0;
+    }
+}
+// An empty string when the library is consistent, else what is wrong with it.
+std::string validate_library(const bepucuda_shape_library& l) {
+    char msg[256];
+    const struct { const void* ptr; int64_t count; const char* name; } arrays[] = {
+        {l.spheres, l.sphere_count, "spheres"}, {l.capsules, l.capsule_count, "capsules"}, {l.boxes, l.box_count, "boxes"}, {l.triangles, l.triangle_count, "triangles"},
+        {l.cylinders, l.cylinder_count, "cylinders"}, {l.hull_points, l.hull_bundle_total, "hull_points"}, {l.hulls, l.hull_count, "hulls"},
+        {l.compound_children, l.compound_child_total, "compound_children"}, {l.compounds, l.compound_count, "compounds"}, {l.big_compounds, l.big_compound_count, "big_compounds"},
+        {l.mesh_triangles, l.mesh_triangle_total, "mesh_triangles"}, {l.meshes, l.mesh_count, "meshes"}};
+    for (const auto& a : arrays) {
+        if (a.count < 0) return std::string(a.name) + ": negative count";
+        if (a.count > 0 && !a.ptr) return std::string(a.name) + ": null pointer with a non-zero count";
+    }
+    for (int t = 0; t <= 8; ++t)
+        if (library_count(l, t) > (1 << 24)) return "shape type " + std::to_string(t) + ": more entries than a TypedIndex can address (2^24)";
+    if ((l.hull_count > 0 || l.hull_bundle_total > 0) && !(l.hull_bundle_width == 4 || l.hull_bundle_width == 8 || l.hull_bundle_width == 16))
+        return "hull_bundle_width must be 4, 8 or 16 (Vector<float>.Count)";
+    for (int64_t i = 0; i < l.hull_count; ++i) {
+        const bepucuda_hull h = l.hulls[i];
+        if (h.bundle_count < 1) return (snprintf(msg, sizeof msg, "hull %lld is empty", (long long)i), msg);
+        if (h.first_bundle < 0 || (int64_t)h.first_bundle + h.bundle_count > l.hull_bundle_total)
+            return (snprintf(msg, sizeof msg, "hull %lld: bundles [%d, %lld) outside hull_points (%lld bundles)", (long long)i, h.first_bundle, (long long)h.first_bundle + h.bundle_count, (long long)l.hull_bundle_total), msg);
+    }
+    for (int kind = 0; kind < 2; ++kind) {
+        const bepucuda_compound* list = kind ? l.big_compounds : l.compounds;
+        const int64_t count = kind ? l.big_compound_count : l.compound_count;
+        const char* name = kind ? "big compound" : "compound";
+        for (int64_t i = 0; i < count; ++i) {
+            const bepucuda_compound c = list[i];
+            if (c.child_count < 1) return (snprintf(msg, sizeof msg, "%s %lld is empty", name, (long long)i), msg);
+            if (c.first_child < 0 || (int64_t)c.first_child + c.child_count > l.compound_child_total)
+                return (snprintf(msg, sizeof msg, "%s %lld: children [%d, %lld) outside compound_children (%lld)", name, (long long)i, c.first_child, (long long)c.first_child + c.child_count, (long long)l.compound_child_total), msg);
+        }
+    }
+    for (int64_t i = 0; i < l.compound_child_total; ++i) {
+        const uint32_t shape = l.compound_children[i].shape;
+        const int32_t type = (int32_t)((shape & 0x7F000000u) >> 24), index = (int32_t)(shape & 0x00FFFFFFu);
+        if (!(shape & 0x80000000u) || type > 5)
+            return (snprintf(msg, sizeof msg, "compound child %lld: shape 0x%08x is not an existing convex shape (types 0-5)", (long long)i, shape), msg);
+        if (index >= library_count(l, type))
+            return (snprintf(msg, sizeof msg, "compound child %lld: index %d out of range for shape type %d (%lld)", (long long)i, index, type, (long long)library_count(l, type)), msg);
+    }
+    for (int64_t i = 0; i < l.mesh_count; ++i) {
+        const bepucuda_mesh m = l.meshes[i];
+        if (m.triangle_count < 1) return (snprintf(msg, sizeof msg, "mesh %lld is empty", (long long)i), msg);
+        if (m.first_triangle < 0 || m.first_triangle + m.triangle_count > l.mesh_triangle_total)
+            return (snprintf(msg, sizeof msg, "mesh %lld: triangles [%lld, %lld) outside mesh_triangles (%lld)", (long long)i, (long long)m.first_triangle, (long long)(m.first_triangle + m.triangle_count), (long long)l.mesh_triangle_total), msg);
+    }
+    return "";
+}
+}  // namespace
+
+int32_t bepucuda_set_shape_library(bepucuda_ctx* ctx, const bepucuda_shape_library* library) {
+    if (!ctx || !library) return fail(ctx, BEPUCUDA_ERR_INVALID_ARGUMENT, "set_shape_library: bad arguments");
+    const bepucuda_shape_library& l = *library;
+    const std::string problem = validate_library(l);
+    if (!problem.empty()) return fail(ctx, BEPUCUDA_ERR_INVALID_ARGUMENT, "set_shape_library: " + problem);
+    CK(cudaSetDevice(ctx->device));
+    auto& sb = ctx->shape_bounds;
+    sb.library_set = false;
+    sb.active = false;  // the work lists index the old library
+    sb.collidable_count = -1;
+    const int64_t w = l.hull_bundle_width;
+    const struct { const void* ptr; size_t bytes; } arrays[12] = {
+        {l.spheres, (size_t)l.sphere_count * 4}, {l.capsules, (size_t)l.capsule_count * 8}, {l.boxes, (size_t)l.box_count * 12}, {l.triangles, (size_t)l.triangle_count * 36},
+        {l.cylinders, (size_t)l.cylinder_count * 8}, {l.hull_points, (size_t)l.hull_bundle_total * 12 * (size_t)w}, {l.hulls, (size_t)l.hull_count * sizeof(bepucuda_hull)},
+        {l.compound_children, (size_t)l.compound_child_total * sizeof(bepucuda_compound_child)}, {l.compounds, (size_t)l.compound_count * sizeof(bepucuda_compound)},
+        {l.big_compounds, (size_t)l.big_compound_count * sizeof(bepucuda_compound)}, {l.mesh_triangles, (size_t)l.mesh_triangle_total * 36},
+        {l.meshes, (size_t)l.mesh_count * sizeof(bepucuda_mesh)}};
+    for (int k = 0; k < 12; ++k) {
+        CK(sb.library[k].reserve(std::max<size_t>(arrays[k].bytes, 16)));
+        if (arrays[k].bytes) CK(cudaMemcpyAsync(sb.library[k].ptr, arrays[k].ptr, arrays[k].bytes, cudaMemcpyHostToDevice, ctx->stream));
+    }
+    CK(cudaStreamSynchronize(ctx->stream));  // the caller's buffers are only guaranteed for the duration of the call
+    ShapeLibraryView& v = sb.view;
+    v.spheres = sb.library[0].as<float>(), v.capsules = sb.library[1].as<float>(), v.boxes = sb.library[2].as<float>(), v.triangles = sb.library[3].as<float>();
+    v.cylinders = sb.library[4].as<float>(), v.hull_points = sb.library[5].as<float>(), v.hulls = sb.library[6].as<bepu_bounds_math::HullRecord>();
+    v.compound_children = sb.library[7].as<bepu_bounds_math::CompoundChildRecord>(), v.compounds = sb.library[8].as<bepu_bounds_math::CompoundRecord>();
+    v.big_compounds = sb.library[9].as<bepu_bounds_math::CompoundRecord>(), v.mesh_triangles = sb.library[10].as<float>(), v.meshes = sb.library[11].as<bepu_bounds_math::MeshRecord>();
+    v.hull_width = (int32_t)w;
+    sb.counts = l;
+    sb.counts.spheres = sb.counts.capsules = sb.counts.boxes = sb.counts.triangles = sb.counts.cylinders = sb.counts.hull_points = sb.counts.mesh_triangles = nullptr;
+    sb.counts.hulls = nullptr, sb.counts.compound_children = nullptr, sb.counts.compounds = sb.counts.big_compounds = nullptr, sb.counts.meshes = nullptr;
+    sb.meshes.assign(l.meshes, l.meshes + l.mesh_count);
+    sb.library_set = true;
+    return BEPUCUDA_OK;
+}
+
+int32_t bepucuda_set_body_collidables(bepucuda_ctx* ctx, const bepucuda_body_collidable* collidables, int32_t body_count) {
+    if (!ctx || body_count < 0 || (body_count > 0 && !collidables)) return fail(ctx, BEPUCUDA_ERR_INVALID_ARGUMENT, "set_body_collidables: bad arguments");
+    auto& sb = ctx->shape_bounds;
+    if (!sb.library_set) return fail(ctx, BEPUCUDA_ERR_BAD_STATE, "set_body_collidables: bepucuda_set_shape_library was not called");
+    // per-class work lists; every built-in index is checked against the library
+    std::vector<int32_t> hulls, compounds;
+    std::vector<MeshBody> mesh_bodies;
+    std::vector<MeshChunk> chunks;
+    for (int32_t i = 0; i < body_count; ++i) {
+        const uint32_t shape = collidables[i].shape;
+        const int32_t type = (int32_t)((shape & 0x7F000000u) >> 24), index = (int32_t)(shape & 0x00FFFFFFu);
+        if (!(shape & 0x80000000u) || type > 8) continue;  // no shape / user-registered type: valid = 0
+        if (index >= library_count(sb.counts, type)) {
+            char msg[160];
+            snprintf(msg, sizeof msg, "set_body_collidables: body %d: index %d out of range for shape type %d (%lld in the library)", i, index, type, (long long)library_count(sb.counts, type));
+            return fail(ctx, BEPUCUDA_ERR_INVALID_ARGUMENT, msg);
+        }
+        if (type == 5) hulls.push_back(i);
+        else if (type == 6 || type == 7) compounds.push_back(i);
+        else if (type == 8) {
+            const bepucuda_mesh& m = sb.meshes[index];
+            MeshBody mb{i, index, (int32_t)chunks.size(), 0};
+            for (int64_t t = 0; t < m.triangle_count; t += kMeshChunkTriangles, ++mb.chunk_count)
+                chunks.push_back(MeshChunk{m.first_triangle + t, (int32_t)std::min<int64_t>(kMeshChunkTriangles, m.triangle_count - t), (int32_t)mesh_bodies.size()});
+            mesh_bodies.push_back(mb);
+        }
+    }
+    CK(cudaSetDevice(ctx->device));
+    auto upload = [&](DeviceBuffer& buf, const void* src, size_t bytes) -> cudaError_t {
+        cudaError_t e = buf.reserve(std::max<size_t>(bytes, 16));
+        if (e == cudaSuccess && bytes) e = cudaMemcpyAsync(buf.ptr, src, bytes, cudaMemcpyHostToDevice, ctx->stream);
+        return e;
+    };
+    CK(upload(sb.collidables, collidables, (size_t)body_count * sizeof(bepucuda_body_collidable)));
+    CK(upload(sb.hull_bodies, hulls.data(), hulls.size() * sizeof(int32_t)));
+    CK(upload(sb.compound_bodies, compounds.data(), compounds.size() * sizeof(int32_t)));
+    CK(upload(sb.mesh_bodies, mesh_bodies.data(), mesh_bodies.size() * sizeof(MeshBody)));
+    CK(upload(sb.mesh_chunks, chunks.data(), chunks.size() * sizeof(MeshChunk)));
+    CK(sb.mesh_partials.reserve(std::max<size_t>(chunks.size() * 6 * sizeof(float), 16)));
+    CK(cudaStreamSynchronize(ctx->stream));
+    ShapeBoundsWork& w = sb.work;
+    w.collidables = sb.collidables.as<BodyCollidableRecord>();
+    w.hull_bodies = sb.hull_bodies.as<int32_t>(), w.hull_body_count = (int32_t)hulls.size();
+    w.compound_bodies = sb.compound_bodies.as<int32_t>(), w.compound_body_count = (int32_t)compounds.size();
+    w.mesh_bodies = sb.mesh_bodies.as<MeshBody>(), w.mesh_body_count = (int32_t)mesh_bodies.size();
+    w.mesh_chunks = sb.mesh_chunks.as<MeshChunk>(), w.mesh_chunk_count = (int32_t)chunks.size();
+    w.mesh_partials = sb.mesh_partials.as<float>();
+    sb.collidable_count = body_count;
+    sb.active = true;
     return BEPUCUDA_OK;
 }
 

@@ -98,6 +98,7 @@ C_ABI_SYMBOLS = [
     "bepucuda_set_contact_features", "bepucuda_update_contacts", "bepucuda_upload_body_motion", "bepucuda_download_body_motion",
     "bepucuda_shard_export", "bepucuda_shard_import", "bepucuda_shard_set_global", "bepucuda_shard_set_pushes", "bepucuda_shard_set_body_masks", "bepucuda_shard_import_contexts",
     "bepucuda_color_constraints", "bepucuda_color_hash", "bepucuda_set_body_shapes", "bepucuda_predict_bounding_boxes",
+    "bepucuda_set_shape_library", "bepucuda_set_body_collidables",
 ]
 
 
@@ -107,6 +108,64 @@ BODY_SHAPE_DTYPE = np.dtype([("type", "<i4"), ("a", "<f4"), ("b", "<f4"), ("c", 
 BODY_ACTIVITY_DTYPE = np.dtype([("sleep_threshold", "<f4"), ("minimum_timesteps_under_threshold", "u1"), ("timesteps_under_threshold_count", "u1"), ("sleep_candidate", "u1"),
                                 ("reserved", "u1")])
 SHAPE_SPHERE, SHAPE_CAPSULE, SHAPE_BOX, SHAPE_CYLINDER = 0, 1, 2, 4  # Sphere.Id, Capsule.Id, Box.Id, Cylinder.Id of the reference
+SHAPE_TRIANGLE, SHAPE_CONVEX_HULL, SHAPE_COMPOUND, SHAPE_BIG_COMPOUND, SHAPE_MESH = 3, 5, 6, 7, 8
+
+# bepucuda_shape_library's record types and bepucuda_body_collidable (include/bepucuda.h)
+HULL_DTYPE = np.dtype([("first_bundle", "<i4"), ("bundle_count", "<i4")])
+COMPOUND_DTYPE = np.dtype([("first_child", "<i4"), ("child_count", "<i4")])
+COMPOUND_CHILD_DTYPE = np.dtype([("local_orientation", "<f4", 4), ("local_position", "<f4", 3), ("shape", "<u4")])  # CompoundChild, 32 B
+MESH_DTYPE = np.dtype([("first_triangle", "<i8"), ("triangle_count", "<i4"), ("scale", "<f4", 3)])
+BODY_COLLIDABLE_DTYPE = np.dtype([("shape", "<u4"), ("minimum_speculative_margin", "<f4"), ("maximum_speculative_margin", "<f4"),
+                                  ("allow_expansion_beyond_speculative_margin", "<i4")])
+
+
+def typed_index(shape_type, index):
+    """TypedIndex.Packed (TypedIndex.cs:L45-51): bit 31 set, type in bits 24-30, index in bits 0-23. Works elementwise on arrays."""
+    return ((np.asarray(shape_type, dtype=np.uint32) << np.uint32(24)) | np.asarray(index, dtype=np.uint32) | np.uint32(1 << 31)).astype(np.uint32)
+
+
+class ShapeLibraryDesc(C.Structure):
+    """bepucuda_shape_library."""
+    _fields_ = [(n, C.c_void_p) for n in ("spheres", "capsules", "boxes", "triangles", "cylinders", "hull_points", "hulls", "compound_children", "compounds", "big_compounds",
+                                          "mesh_triangles", "meshes")] + \
+               [(n, C.c_int64) for n in ("sphere_count", "capsule_count", "box_count", "triangle_count", "cylinder_count", "hull_bundle_width", "hull_bundle_total", "hull_count",
+                                         "compound_child_total", "compound_count", "big_compound_count", "mesh_triangle_total", "mesh_count")]
+
+
+class ShapeLibrary:
+    """The reference's Shapes batches, flattened as bepucuda_set_shape_library takes them. Primitive batches are float arrays of one record per
+    shape: spheres [n] (Radius), capsules [n, 2] (Radius, HalfLength), boxes [n, 3], triangles [n, 9] (A, B, C), cylinders [n, 2]. hull_points
+    [bundles, 3, W] holds the Vector3Wide bundles of every hull (ConvexHull.Points), hulls / compounds / big_compounds / meshes are HULL_DTYPE /
+    COMPOUND_DTYPE / MESH_DTYPE records indexing hull_points / compound_children (COMPOUND_CHILD_DTYPE) / mesh_triangles [n, 9]."""
+
+    def __init__(self, spheres=(), capsules=(), boxes=(), triangles=(), cylinders=(), hull_points=None, hull_bundle_width=8, hulls=(), compound_children=(),
+                 compounds=(), big_compounds=(), mesh_triangles=(), meshes=()):
+        f = lambda a, k: np.ascontiguousarray(np.asarray(a, dtype=np.float32).reshape(-1, k) if k > 1 else np.asarray(a, dtype=np.float32).reshape(-1))
+        self.spheres, self.capsules, self.boxes, self.triangles, self.cylinders = f(spheres, 1), f(capsules, 2), f(boxes, 3), f(triangles, 9), f(cylinders, 2)
+        self.hull_bundle_width = int(hull_bundle_width)
+        self.hull_points = np.ascontiguousarray(np.zeros((0, 3, self.hull_bundle_width), np.float32) if hull_points is None else np.asarray(hull_points, dtype=np.float32))
+        r = lambda a, dtype: np.ascontiguousarray(np.zeros(0, dtype) if len(a) == 0 else a.astype(dtype) if isinstance(a, np.ndarray) else np.array(list(a), dtype=dtype)).reshape(-1)
+        self.hulls = r(hulls, HULL_DTYPE)
+        self.compound_children = r(compound_children, COMPOUND_CHILD_DTYPE)
+        self.compounds, self.big_compounds = r(compounds, COMPOUND_DTYPE), r(big_compounds, COMPOUND_DTYPE)
+        self.mesh_triangles = f(mesh_triangles, 9)
+        self.meshes = r(meshes, MESH_DTYPE)
+
+    def desc(self):
+        """The bepucuda_shape_library pointing into this object's arrays (valid while the object lives)."""
+        d = ShapeLibraryDesc()
+        for name in ("spheres", "capsules", "boxes", "triangles", "cylinders", "hull_points", "hulls", "compound_children", "compounds", "big_compounds", "mesh_triangles", "meshes"):
+            a = getattr(self, name)
+            setattr(d, name, a.ctypes.data if a.size else None)
+        d.sphere_count, d.capsule_count, d.box_count = len(self.spheres), len(self.capsules), len(self.boxes)
+        d.triangle_count, d.cylinder_count = len(self.triangles), len(self.cylinders)
+        d.hull_bundle_width, d.hull_bundle_total, d.hull_count = self.hull_bundle_width, self.hull_points.shape[0], len(self.hulls)
+        d.compound_child_total, d.compound_count, d.big_compound_count = len(self.compound_children), len(self.compounds), len(self.big_compounds)
+        d.mesh_triangle_total, d.mesh_count = len(self.mesh_triangles), len(self.meshes)
+        return d
+
+    def count(self, shape_type):
+        return len([self.spheres, self.capsules, self.boxes, self.triangles, self.cylinders, self.hulls, self.compounds, self.big_compounds, self.meshes][shape_type])
 
 EXCHANGE_FN = C.CFUNCTYPE(C.c_int32, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p)
 
@@ -163,6 +222,8 @@ def load_libraries():
     cuda.bepucuda_color_hash.argtypes = [C.c_uint32]
     cuda.bepucuda_set_body_shapes.argtypes = [vp, vp, i32]
     cuda.bepucuda_predict_bounding_boxes.argtypes = [vp, f32, vp, vp]
+    cuda.bepucuda_set_shape_library.argtypes = [vp, C.POINTER(ShapeLibraryDesc)]
+    cuda.bepucuda_set_body_collidables.argtypes = [vp, vp, i32]
     cuda.bepucuda_color_hash.restype = C.c_uint32
 
     host.bepuhost_create.restype = vp
@@ -392,6 +453,16 @@ class CudaTimestepper:
         """bepucuda_set_body_shapes: one BODY_SHAPE_DTYPE record per body (static between frames unless a shape changes)."""
         shapes = np.ascontiguousarray(shapes, dtype=BODY_SHAPE_DTYPE)
         self._check(self._cuda.bepucuda_set_body_shapes(self._ctx, shapes.ctypes.data, shapes.shape[0]))
+
+    def set_shape_library(self, library):
+        """bepucuda_set_shape_library: uploads a ShapeLibrary (once; again when shapes change, followed by set_body_collidables)."""
+        desc = library.desc()
+        self._check(self._cuda.bepucuda_set_shape_library(self._ctx, C.byref(desc)))
+
+    def set_body_collidables(self, collidables):
+        """bepucuda_set_body_collidables: one BODY_COLLIDABLE_DTYPE record per body; from now on predict_bounding_boxes covers every built-in shape type."""
+        collidables = np.ascontiguousarray(collidables, dtype=BODY_COLLIDABLE_DTYPE)
+        self._check(self._cuda.bepucuda_set_body_collidables(self._ctx, collidables.ctypes.data if collidables.size else None, collidables.shape[0]))
 
     def predict_bounding_boxes(self, dt, activities):
         """bepucuda_predict_bounding_boxes on the body state resident on the device. `activities` (BODY_ACTIVITY_DTYPE) is updated in place.

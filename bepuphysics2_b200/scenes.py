@@ -653,3 +653,92 @@ def build(scene, simulation):
     for type_id, handles, prestep in scene["constraints"]:
         simulation.add_constraints(type_id, handles, prestep)
     return simulation
+
+
+# ---- PredictBoundingBoxes worlds: every built-in shape type (bepucuda_set_shape_library / bepucuda_set_body_collidables) -----------------------
+def bundle_hull_points(points, width):
+    """ConvexHull.Points for a point set: Vector3Wide bundles [bundles, 3, width], the last bundle padded by repeating the last point
+    (ConvexHullHelper.cs:L1050-1062). The bounds only read the points, so any point set will do; it need not be a hull."""
+    points = np.asarray(points, dtype=np.float32).reshape(-1, 3)
+    bundles = (points.shape[0] + width - 1) // width
+    index = np.minimum(np.arange(bundles * width), points.shape[0] - 1)
+    return np.ascontiguousarray(points[index].reshape(bundles, width, 3).transpose(0, 2, 1))
+
+
+def shape_library(rng, hull_width=8, primitives=64, hulls=32, hull_points=(20, 64), compounds=32, big_compounds=8, compound_children=(2, 16), mesh_triangle_counts=(),
+                  mesh_triangles_shared=None):
+    """A random shape library: `primitives` shapes of each primitive type and triangles, hulls of hull_points[0]..[1] points, compounds and big
+    compounds of compound_children[0]..[1] children of every convex type (hulls included), one mesh per entry of mesh_triangle_counts with a
+    non-uniform scale."""
+    from .native import ShapeLibrary, COMPOUND_CHILD_DTYPE, typed_index
+
+    u = lambda lo, hi, *shape: rng.uniform(lo, hi, size=shape).astype(np.float32)
+    bundles, hull_records, first = [], [], 0
+    for _ in range(hulls):
+        pts = bundle_hull_points(u(-1.5, 1.5, int(rng.integers(hull_points[0], hull_points[1] + 1)), 3), hull_width)
+        bundles.append(pts)
+        hull_records.append((first, pts.shape[0]))
+        first += pts.shape[0]
+    counts = {0: primitives, 1: primitives, 2: primitives, 3: primitives, 4: primitives, 5: hulls}
+    children, records = [], [[], []]
+    for kind, how_many in ((0, compounds), (1, big_compounds)):
+        for _ in range(how_many):
+            k = int(rng.integers(compound_children[0], compound_children[1] + 1))
+            c = np.zeros(k, dtype=COMPOUND_CHILD_DTYPE)
+            q = rng.normal(size=(k, 4))
+            c["local_orientation"] = q / np.linalg.norm(q, axis=1, keepdims=True)
+            c["local_position"] = u(-3, 3, k, 3)
+            types = rng.choice([t for t in range(6) if counts[t] > 0], size=k)
+            c["shape"] = typed_index(types, [int(rng.integers(0, counts[t])) for t in types])
+            records[kind].append((sum(len(x) for x in children), k))
+            children.append(c)
+    mesh_pool, mesh_records = [], []
+    for count in mesh_triangle_counts:
+        tri = mesh_triangles_shared[:count] if mesh_triangles_shared is not None else u(-4, 4, count, 9)
+        mesh_records.append((sum(len(x) for x in mesh_pool), count, tuple(u(0.2, 3.0, 3))))
+        mesh_pool.append(tri)
+    return ShapeLibrary(spheres=u(0.05, 2, primitives), capsules=u(0.05, 2, primitives, 2), boxes=u(0.05, 2, primitives, 3), triangles=u(-2, 2, primitives, 9),
+                        cylinders=u(0.05, 2, primitives, 2), hull_points=np.concatenate(bundles) if bundles else None, hull_bundle_width=hull_width, hulls=hull_records,
+                        compound_children=np.concatenate(children) if children else (), compounds=records[0], big_compounds=records[1],
+                        mesh_triangles=np.concatenate(mesh_pool) if mesh_pool else (), meshes=mesh_records)
+
+
+def shape_world(body_count, seed=5, library=None, type_weights=None, kinematic_fraction=0.1, **library_args):
+    """Random bodies over a shape library (shape_library(**library_args) unless one is given): BodyDynamics records, one BODY_COLLIDABLE_DTYPE
+    and one BODY_ACTIVITY_DTYPE record per body. type_weights: relative frequency of the shape types 0-8, plus 'none' (no shape) and 'user'
+    (a user-registered type id, which has no built-in bounds). Spins range from still to fast enough for the pi/3 clamp."""
+    from .native import BODY_ACTIVITY_DTYPE, BODY_COLLIDABLE_DTYPE, typed_index
+
+    rng = np.random.default_rng(seed)
+    library = library if library is not None else shape_library(rng, **library_args)
+    weights = dict(type_weights or {0: 1, 1: 1, 2: 1, 3: 1, 4: 1, 5: 2, 6: 2, 7: 1, 8: 0.2, "none": 0.3, "user": 0.2})
+    for t in list(weights):
+        if isinstance(t, int) and library.count(t) == 0:
+            weights.pop(t)
+    keys = list(weights)
+    p = np.array([weights[k] for k in keys], dtype=np.float64)
+    kinds = rng.choice(len(keys), size=body_count, p=p / p.sum())
+    collidables = np.zeros(body_count, dtype=BODY_COLLIDABLE_DTYPE)
+    for j, k in enumerate(keys):
+        sel = kinds == j
+        m = int(sel.sum())
+        if k == "none":
+            collidables["shape"][sel] = rng.integers(0, 1 << 31, size=m).astype(np.uint32) & np.uint32(0x7FFFFFFF)
+        elif k == "user":
+            collidables["shape"][sel] = typed_index(rng.integers(9, 128, size=m), rng.integers(0, 1 << 24, size=m))
+        else:
+            collidables["shape"][sel] = typed_index(np.full(m, k), rng.integers(0, library.count(k), size=m))
+    collidables["minimum_speculative_margin"] = rng.choice([0.0, 0.01, 0.2], size=body_count)
+    collidables["maximum_speculative_margin"] = rng.choice([0.05, 1.0, 3.40282347e+38], size=body_count)
+    collidables["allow_expansion_beyond_speculative_margin"] = rng.integers(0, 2, size=body_count)
+    q = _random_unit_quaternions(rng, body_count)
+    bodies = make_bodies(rng.uniform(-50, 50, size=(body_count, 3)), orientation=q,
+                         linear=rng.normal(size=(body_count, 3)) * rng.choice([0.0, 0.1, 5.0, 80.0], size=(body_count, 1)),
+                         angular=rng.normal(size=(body_count, 3)) * rng.choice([0.0, 0.3, 10.0, 200.0], size=(body_count, 1)),
+                         inverse_mass=np.ones(body_count), inverse_inertia=np.tile(np.array([[1, 0, 1, 0, 0, 1]], dtype=np.float32), (body_count, 1)))
+    bodies[rng.random(body_count) < kinematic_fraction, 16:23] = 0.0
+    activities = np.zeros(body_count, dtype=BODY_ACTIVITY_DTYPE)
+    activities["sleep_threshold"] = rng.choice([-1.0, 0.01, 5.0], size=body_count)
+    activities["minimum_timesteps_under_threshold"] = rng.integers(1, 40, size=body_count)
+    activities["timesteps_under_threshold_count"] = rng.integers(0, 256, size=body_count)
+    return {"bodies": bodies, "library": library, "collidables": collidables, "activities": activities}

@@ -200,8 +200,8 @@ int32_t bepucuda_profile_stages(bepucuda_ctx* ctx, float dt, bepucuda_stage_prof
  * margin BoundingBoxBatcher.ExecuteConvexBatch computes (Collidables/BoundingBoxBatcher.cs:L142-222; IConvexShape.GetBounds of Sphere.cs:L149-160,
  * Capsule.cs:L226-239, Box.cs:L211-222, Cylinder.cs:L222-235; BoundingBoxHelpers.cs:L12-58).
  *   bepucuda_body_shape.type: the reference's shape type id -- 0 sphere (a = radius), 1 capsule (a = radius, b = half length), 2 box (a, b, c = half
- *   width, height, length), 4 cylinder (a = radius, b = half length). Any other value (no shape; triangle, hull, compound, mesh: their bounds stay
- *   on the host) yields valid = 0 for that body; its activity is still updated.
+ *   width, height, length), 4 cylinder (a = radius, b = half length). Any other value (no shape; triangle, hull, compound, mesh) yields valid = 0
+ *   for that body; its activity is still updated. bepucuda_set_shape_library + bepucuda_set_body_collidables below cover every built-in type.
  *   bepucuda_body_activity = BodyActivity (BodyProperties.cs:L386-416), updated in place.
  *   bounds_out: 8 floats per body {min.x, min.y, min.z, speculative margin, max.x, max.y, max.z, valid (1 or 0)}.
  * Uses the body arrays as they are on the device (after bepucuda_upload_bodies / bepucuda_solve) and the integrator set by bepucuda_set_integrator.
@@ -223,6 +223,77 @@ typedef struct bepucuda_body_activity {
 } bepucuda_body_activity;
 int32_t bepucuda_set_body_shapes(bepucuda_ctx* ctx, const bepucuda_body_shape* shapes, int32_t body_count);
 int32_t bepucuda_predict_bounding_boxes(bepucuda_ctx* ctx, float dt, bepucuda_body_activity* activities, float* bounds_out);
+
+/* PredictBoundingBoxes for every built-in shape type: the reference's Shapes batches are uploaded once as a library, and each active body names its
+ * shape with the reference's TypedIndex. Whichever of bepucuda_set_body_shapes / bepucuda_set_body_collidables was called last decides what
+ * bepucuda_predict_bounding_boxes computes; its signature, its activity update and its output format are the same for both.
+ *   Sphere (0), Capsule (1), Box (2), Cylinder (4) and Triangle (3, TriangleWide.GetBounds, Collidables/Triangle.cs:L203-221) and ConvexHull (5,
+ *   ConvexHullWide.GetBounds, ConvexHull.cs:L319-364) go through ExecuteConvexBatch (Collidables/BoundingBoxBatcher.cs:L142-223). Compound (6) and
+ *   BigCompound (7) go through ExecuteCompoundBatch (L268-287) and Compound.AddChildBoundsToBatcher (Compound.cs:L198-221): every child is bounded
+ *   like a convex body with the parent's margins and the child's pose and velocity, and the children's boxes and margins are merged. Mesh (8)
+ *   goes through ExecuteHomogeneousCompoundBatch (L225-266) and Mesh.ComputeBounds (Mesh.cs:L232-255).
+ *   Results are bit-identical to a non-contracting fp32 evaluation of the reference's expressions, including the sign of a zero that ties in a
+ *   min / max fold, with one documented exception: the reference merges a compound's children in the order its batcher flushes them (grouped by
+ *   child type, 16 per flush, shared across bodies), which depends on the other bodies of the frame; this library merges them in child order. The
+ *   two agree except for the sign of a zero coordinate on which two children tie.
+ *   A body whose shape does not exist (bit 31 of the TypedIndex clear) or has a type id above 8 (a user-registered shape) gets valid = 0; its
+ *   activity is still updated. */
+typedef struct bepucuda_hull {
+    int32_t first_bundle;   /* into hull_points, in bundles */
+    int32_t bundle_count;   /* ConvexHull.Points.Length, >= 1 */
+} bepucuda_hull;
+typedef struct bepucuda_compound {
+    int32_t first_child;    /* into compound_children */
+    int32_t child_count;    /* Compound.Children.Length / BigCompound.Children.Length, >= 1 */
+} bepucuda_compound;
+typedef struct bepucuda_compound_child {  /* CompoundChild (Compound.cs:L18-31), 32 B */
+    float local_orientation[4];           /* Quaternion x, y, z, w */
+    float local_position[3];
+    uint32_t shape;                       /* TypedIndex.Packed; types 0-5 only */
+} bepucuda_compound_child;
+typedef struct bepucuda_mesh {
+    int64_t first_triangle;   /* into mesh_triangles, in triangles */
+    int32_t triangle_count;   /* Mesh.Triangles.Length, >= 1 */
+    float scale[3];           /* Mesh.Scale */
+} bepucuda_mesh;
+/* The shape library. Primitive batches are the reference's ShapeBatch<T>.shapes memory as it is: Sphere {Radius}, Capsule {Radius, HalfLength},
+ * Box {HalfWidth, HalfHeight, HalfLength}, Triangle {A, B, C} (36 B), Cylinder {Radius, HalfLength}; index i of a batch is TypedIndex.Index.
+ * hull_points: the Vector3Wide bundles of every hull back to back (ConvexHull.Points memory: per bundle W x floats, W y floats, W z floats; the
+ * last bundle padded by repeating the last point, ConvexHullHelper.cs:L1050-1062), hull_bundle_width = W = Vector<float>.Count of the process that
+ * built them (4, 8 or 16). compound_children: the children of every compound and big compound back to back. mesh_triangles: the Triangle records
+ * of every mesh back to back. A pointer may be NULL when its count is 0. Host buffers are only read during the call. */
+typedef struct bepucuda_shape_library {
+    const float* spheres;
+    const float* capsules;
+    const float* boxes;
+    const float* triangles;
+    const float* cylinders;
+    const float* hull_points;
+    const bepucuda_hull* hulls;
+    const bepucuda_compound_child* compound_children;
+    const bepucuda_compound* compounds;
+    const bepucuda_compound* big_compounds;
+    const float* mesh_triangles;
+    const bepucuda_mesh* meshes;
+    int64_t sphere_count, capsule_count, box_count, triangle_count, cylinder_count;
+    int64_t hull_bundle_width, hull_bundle_total, hull_count;
+    int64_t compound_child_total, compound_count, big_compound_count;
+    int64_t mesh_triangle_total, mesh_count;
+} bepucuda_shape_library;
+/* One per active body: the reference's Collidable (Collidable.cs:L115-152). */
+typedef struct bepucuda_body_collidable {
+    uint32_t shape;                                     /* TypedIndex.Packed: bit 31 exists, bits 24-30 type, bits 0-23 index */
+    float minimum_speculative_margin;                   /* Collidable.MinimumSpeculativeMargin */
+    float maximum_speculative_margin;                   /* Collidable.MaximumSpeculativeMargin */
+    int32_t allow_expansion_beyond_speculative_margin;  /* Collidable.Continuity.AllowExpansionBeyondSpeculativeMargin */
+} bepucuda_body_collidable;
+/* Validates and uploads the library (index ranges of every hull, compound, child and mesh inside their pools, no empty hull / compound / mesh,
+ * compound children of types 0-5 with indices in range, W in {4, 8, 16} when there are hulls). Call again when shapes change; the body
+ * collidables must then be set again before the next prediction. */
+int32_t bepucuda_set_shape_library(bepucuda_ctx* ctx, const bepucuda_shape_library* library);
+/* Validates every existing built-in shape index against the library and builds the per-class work lists (hulls, compounds, meshes and the
+ * chunks of large meshes). body_count must equal the uploaded body count when bepucuda_predict_bounding_boxes runs. */
+int32_t bepucuda_set_body_collidables(bepucuda_ctx* ctx, const bepucuda_body_collidable* collidables, int32_t body_count);
 
 /* Device-side batch colouring (SURVEY.md §8 f3). Replaces, for a whole constraint set at once, the batch search Solver.Add runs per constraint
  * (Solver.cs:L1182-1199: the first batch whose referenced-handle set holds none of the constraint's dynamic bodies; kinematic references never

@@ -33,6 +33,28 @@ namespace BepuCuda
         public fixed long AlgorithmicBytes[8];
     }
 
+    // bepucuda_set_shape_library / bepucuda_set_body_collidables. The pools are the reference's own memory: ShapeBatch<T>.shapes.Memory for the
+    // primitive batches (Sphere, Capsule, Box, Triangle, Cylinder), ConvexHull.Points, Compound.Children / BigCompound.Children (CompoundChild, 32 B),
+    // Mesh.Triangles; hulls, compounds and meshes are gathered back to back into one pool per kind.
+    [StructLayout(LayoutKind.Sequential)] public struct HullRange { public int FirstBundle, BundleCount; }
+    [StructLayout(LayoutKind.Sequential)] public struct CompoundRange { public int FirstChild, ChildCount; }
+    [StructLayout(LayoutKind.Sequential)]
+    public unsafe struct MeshRange { public long FirstTriangle; public int TriangleCount; public fixed float Scale[3]; }
+    [StructLayout(LayoutKind.Sequential)]
+    public unsafe struct ShapeLibrary
+    {
+        public float* Spheres, Capsules, Boxes, Triangles, Cylinders, HullPoints;
+        public HullRange* Hulls;
+        public void* CompoundChildren;  // BepuPhysics.Collidables.CompoundChild*
+        public CompoundRange* Compounds, BigCompounds;
+        public float* MeshTriangles;
+        public MeshRange* Meshes;
+        public long SphereCount, CapsuleCount, BoxCount, TriangleCount, CylinderCount, HullBundleWidth, HullBundleTotal, HullCount;
+        public long CompoundChildTotal, CompoundCount, BigCompoundCount, MeshTriangleTotal, MeshCount;
+    }
+    [StructLayout(LayoutKind.Sequential)]
+    public struct BodyCollidable { public uint Shape; public float MinimumSpeculativeMargin, MaximumSpeculativeMargin; public int AllowExpansionBeyondSpeculativeMargin; }
+
     [UnmanagedFunctionPointer(CallingConvention.Cdecl)]
     public unsafe delegate int ExchangeFn(void* user, void* deviceWords, long count, int op, void* cudaStream);
 
@@ -75,6 +97,8 @@ namespace BepuCuda
         /// <summary>PredictBoundingBoxes on the device: sleep candidacy + bounds and speculative margins of sphere / capsule / box / cylinder bodies from the resident body state.</summary>
         [DllImport(Lib)] public static extern int bepucuda_set_body_shapes(IntPtr ctx, BodyShape* shapes, int bodyCount);
         [DllImport(Lib)] public static extern int bepucuda_predict_bounding_boxes(IntPtr ctx, float dt, BodyActivity* activities, float* boundsOut);
+        [DllImport(Lib)] public static extern int bepucuda_set_shape_library(IntPtr ctx, ShapeLibrary* library);
+        [DllImport(Lib)] public static extern int bepucuda_set_body_collidables(IntPtr ctx, BodyCollidable* collidables, int bodyCount);
         /// <summary>Device-side batch colouring: the batch Solver.Add's first-fit search would pick for every constraint of a list (order 0 = add order, 1 = hashed, 2 = priorities).</summary>
         [DllImport(Lib)] public static extern int bepucuda_color_constraints(IntPtr ctx, int constraintCount, int bodiesPerConstraint, int* encodedBodyReferences, int bodyCount, int fallbackBatchThreshold, int order, uint* priorities, int* batchIndicesOut, int* batchCountOut, int* roundsOut);
         [DllImport(Lib)] public static extern uint bepucuda_color_hash(uint constraintIndex);
